@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the headline benchmark of the hot path (BASELINE.json).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload metric|cfg2|cfg3|cfg4]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload metric|cfg2|cfg3|cfg4] [--dump-outputs DIR]
 
 metric   Msplats/s (= splat_count / frame time) and ms/frame, full frame = CSCalcDistances + radix sort + CSCalcViewData +
          draw/blend, sorted every frame (m_SortNthFrame = 1), the camera ORBITING the scene by a fixed step per frame (no two
@@ -22,6 +22,11 @@ N > 1    the group path (include/gsplat_b200.h gs_group_*): key-range-sharded de
          view-calc / binning / compositing + one NCCL exchange of the composited rows, all of it issued by the library
          itself.  Before the timed region EVERY rank renders the same frames on its own GPU alone and asserts that the
          group's draw order and render target are bit-identical.
+--dump-outputs DIR  after the timed steps, the render target of the last timed step (what the caller of
+         SortAndRenderSplats receives) goes to DIR/render_target.npy as float32 (h, w, 4).  Above 60 MB a fixed, seeded
+         sample of its pixels goes instead: render_target_pixels.npy (k, 4) and render_target_pixel_index.npy (k,
+         row-major pixel index, float64).  The scene and the camera path are seeded, so two builds run with the same
+         arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -53,6 +58,7 @@ WORKLOADS = {
 # kept for the tools that import this module
 N_SPLATS, WIDTH, HEIGHT, FOV, SEED = 6_131_954, 1200, 797, 39.09651, 0x5EED0002
 ORBIT_STEP_DEG = 0.5
+DUMP_BYTES = 60 * 10**6   # --dump-outputs writes less than 64 MB, .npy headers included
 NCU_SOURCE = ROOT / "profiles" / "r02_kernels.json"   # written by tools/ncu_kernels_json.py from the committed ncu --set full capture
 
 _assets = {}
@@ -161,7 +167,7 @@ class ClockSampler:
 
 
 def cpu_frame(O, asset, fp, threads, width, height, prev_order=None):
-    """One full frame of the CPU restatement; returns seconds per stage and the new order."""
+    """One full frame of the CPU restatement; returns seconds per stage, the new order and the render target."""
     order = np.arange(asset.splatCount, dtype=np.uint32) if prev_order is None else prev_order.copy()
     t0 = time.perf_counter()
     keys = O.calc_distances(asset, fp, order, threads)
@@ -170,9 +176,23 @@ def cpu_frame(O, asset, fp, threads, width, height, prev_order=None):
     t2 = time.perf_counter()
     view = O.calc_view(asset, fp, threads)
     t3 = time.perf_counter()
-    O.render(view, order, width, height, 0, threads)
+    rt = O.render(view, order, width, height, 0, threads)
     t4 = time.perf_counter()
-    return {"distances": t1 - t0, "sort": t2 - t1, "view": t3 - t2, "draw": t4 - t3, "total": t4 - t0}, order
+    return {"distances": t1 - t0, "sort": t2 - t1, "view": t3 - t2, "draw": t4 - t3, "total": t4 - t0}, order, rt
+
+
+def dump_outputs(directory, rt):
+    """--dump-outputs: the render target as float32, or a fixed, seeded sample of its pixels when it exceeds DUMP_BYTES."""
+    d = Path(directory)
+    d.mkdir(parents=True, exist_ok=True)
+    px = np.asarray(rt).reshape(-1, 4).astype(np.float32)
+    if px.nbytes <= DUMP_BYTES:
+        np.save(d / "render_target.npy", px.reshape(np.shape(rt)))
+        return
+    k = DUMP_BYTES // (px.itemsize * 4 + 8)
+    idx = np.sort(np.random.default_rng(0).choice(px.shape[0], k, replace=False))
+    np.save(d / "render_target_pixels.npy", px[idx])
+    np.save(d / "render_target_pixel_index.npy", idx.astype(np.float64))
 
 
 def workload_text(name, n, quality, w, h):
@@ -191,12 +211,12 @@ def run_reference(args):
     n, quality, w, h, fov, seed, _ = WORKLOADS[args.workload]
     asset = get_asset(n, quality, seed)
     warm = max(0, min(args.warmup, 1))
-    steps = max(1, min(args.steps, 3))
+    steps = args.steps
     order = None
     times = []
     for k in range(warm + steps):
         fp, _keep = g.make_frame_params(orbit_camera(k, w, h, fov))
-        t, order = cpu_frame(O, asset, fp, threads, w, h, order)
+        t, order, rt = cpu_frame(O, asset, fp, threads, w, h, order)
         if k >= warm:
             times.append(t)
     t = statistics.mean(x["total"] for x in times)
@@ -206,10 +226,12 @@ def run_reference(args):
             "scaling": "strong", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": {"workload": workload_text(args.workload, n, quality, w, h)},
             "cpu_baseline": {"value": val, "unit": "Msplats/s", "cores": threads, "kind": "port",
-                             "sample": "full frames of the whole workload (steps capped at 3); CPU restatement of the reference's "
+                             "sample": "full frames of the whole workload; CPU restatement of the reference's "
                                        "HLSL -- the reference has no CPU path"},
             "e2e": {"value": val, "unit": "Msplats/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
             "stages_ms": {k: statistics.mean(x[k] for x in times) * 1e3 for k in times[0]}}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, rt)
     print(json.dumps(line))
 
 
@@ -237,8 +259,9 @@ def stage_report(n, quality, w, h, stages, pass_ms, peak, ms_step, nk):
     return rep
 
 
-def measure_single(g, ctx, stream, torch, name, steps, warmup, want_e2e=True):
-    """One GPU, one workload: device-resident value, per-stage times, e2e through host buffers."""
+def measure_single(g, ctx, stream, torch, name, steps, warmup, want_e2e=True, keep_last=False):
+    """One GPU, one workload: device-resident value, per-stage times, e2e through host buffers.  keep_last: also return
+    the render target of the last timed step ("rt_last")."""
     n, quality, w, h, fov, seed, _ = WORKLOADS[name]
     asset = get_asset(n, quality, seed)
     r = g.GaussianSplatRenderer(asset, ctx)
@@ -258,6 +281,7 @@ def measure_single(g, ctx, stream, torch, name, steps, warmup, want_e2e=True):
         torch.cuda.synchronize()
         ms_step = e0.elapsed_time(e1) / steps
         launches = ctx.stage_times().kernel_launches - launches0
+        rt_last = rt_dev.cpu().numpy() if keep_last else None
         # per-stage device times (CUDA events inside the library, same stream), continuing the orbit
         ctx.set_timing(True)
         acc = {}
@@ -289,7 +313,7 @@ def measure_single(g, ctx, stream, torch, name, steps, warmup, want_e2e=True):
             r.async_readback = False
     r.Dispose()
     return {"n": n, "quality": quality, "w": w, "h": h, "ms_step": ms_step, "launches": int(launches), "stages": stages, "pass_ms": pass_ms,
-            "e2e_ms": e2e_ms}
+            "e2e_ms": e2e_ms, "rt_last": rt_last}
 
 
 def main():
@@ -303,7 +327,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-other-configs", action="store_true")
     ap.add_argument("--baseline-partition", action="store_true", help="N > 1: round 1's interleaved bands + torch all-gather instead of the group path")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the last timed step's render target under DIR (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.screen:
         w, h = (int(v) for v in args.screen.lower().split("x"))
         wl = list(WORKLOADS[args.workload]); wl[2], wl[3] = w, h
@@ -334,7 +361,7 @@ def main():
     nk = ncu_kernels()
 
     if world == 1:
-        m = measure_single(g, ctx, stream, torch, args.workload, args.steps, args.warmup)
+        m = measure_single(g, ctx, stream, torch, args.workload, args.steps, args.warmup, keep_last=bool(args.dump_outputs))
         sampler = ClockSampler(local)
         # clocks: sampled over a second pass of the device-resident loop (the sampler's start-up would otherwise miss a 50 ms region)
         sampler.start()
@@ -365,7 +392,7 @@ def main():
             from oracle import gs_oracle_py as O
             threads = host_threads()
             fp, _keep = g.make_frame_params(orbit_camera(0, W, H, fov))
-            ct, _ = cpu_frame(O, get_asset(n, quality, seed), fp, threads, W, H)
+            ct, _, _ = cpu_frame(O, get_asset(n, quality, seed), fp, threads, W, H)
             cpu = {"value": n / ct["total"] / 1e6, "unit": "Msplats/s", "cores": threads, "kind": "port",
                    "sample": "one full frame of the same workload (%.1f s): distances %.0f ms, sort %.0f ms, view %.0f ms, draw %.0f ms"
                              % (ct["total"], ct["distances"] * 1e3, ct["sort"] * 1e3, ct["view"] * 1e3, ct["draw"] * 1e3)}
@@ -383,6 +410,8 @@ def main():
             "roofline": roofline, "stages": stages, "ncu_source": str(NCU_SOURCE.relative_to(ROOT)) if nk else None,
             "other_configs": others, "cpu_baseline": cpu,
         }
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, m["rt_last"])
         print(json.dumps(line))
         return
 
@@ -448,6 +477,7 @@ def main():
         e1.record(stream)
         barrier()
         ms_total = e0.elapsed_time(e1)
+        rt_last = rt_dev.cpu().numpy() if args.dump_outputs and rank == 0 else None
         clocks = sampler.stop() if rank == 0 else None
         launches = ctx.stage_times().kernel_launches - lib_launch0
         t = torch.tensor([ms_total], device=dev)
@@ -537,6 +567,8 @@ def main():
                 "d2h_bytes_per_step": W * H * 8},
         "roofline": roofline, "stages": stages, "cpu_baseline": None,
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, rt_last)
     print(json.dumps(line))
     dist.destroy_process_group()
 

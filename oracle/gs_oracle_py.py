@@ -7,7 +7,6 @@ from __future__ import annotations
 
 import ctypes as C
 import subprocess
-import sys
 from pathlib import Path
 
 import numpy as np
@@ -203,13 +202,12 @@ _ref_hlsl = None
 
 
 def ref_hlsl():
-    """Loads (building first when /root/reference is present) the compiled-reference library; None when neither exists."""
+    """Loads the compiled-reference library, built by oracle/refhlsl/build_ref_hlsl.py from a checkout of the reference.
+    Only tests/golden/make_ref_hlsl_golden.py needs it; the tests read what it computed from tests/golden/ref_hlsl.npz."""
     global _ref_hlsl
     if _ref_hlsl is None:
-        if Path("/root/reference/package/Shaders").exists():
-            subprocess.run([sys.executable, str(HERE / "refhlsl" / "build_ref_hlsl.py")], check=True, stdout=subprocess.PIPE, stderr=subprocess.STDOUT)
         if not REF_HLSL_LIB.exists():
-            return None
+            raise FileNotFoundError("%s is missing: run oracle/refhlsl/build_ref_hlsl.py <reference checkout>" % REF_HLSL_LIB)
         L = C.CDLL(str(REF_HLSL_LIB))
         L.refhlsl_calc_distances.restype, L.refhlsl_calc_distances.argtypes = C.c_int, [C.POINTER(GsoAsset), C.POINTER(GsoFrame), C.c_void_p, C.c_void_p]
         L.refhlsl_calc_view.restype, L.refhlsl_calc_view.argtypes = C.c_int, [C.POINTER(GsoAsset), C.POINTER(GsoFrame), C.c_void_p]

@@ -1,9 +1,11 @@
 #!/usr/bin/env python
 """Builds oracle/_ref/libref_hlsl.so: the REFERENCE'S OWN shader source, compiled for the CPU.
 
+  python oracle/refhlsl/build_ref_hlsl.py <checkout of aras-p/UnityGaussianSplatting> [--keep]
+
 Recipe (TEST INFRASTRUCTURE; nothing here is product code, nothing of the reference is copied into the repo):
   1. read package/Shaders/{GaussianSplatting.hlsl, SphericalHarmonics.hlsl, SplatUtilities.compute,
-     RenderGaussianSplats.shader} where they lie under /root/reference;
+     RenderGaussianSplats.shader} of the reference checkout named on the command line;
   2. apply the purely syntactic rewrites below (HLSL-only syntax -> C++ spelling; no expression is touched):
        - drop #pragma / #include lines, [numthreads(..)] attributes and `: SEMANTIC` annotations,
        - `out T x` / `inout T x` parameters -> `T& x`,
@@ -14,7 +16,8 @@ Recipe (TEST INFRASTRUCTURE; nothing here is product code, nothing of the refere
   3. write the result to oracle/_ref/ref_cs.inc and ref_ps.inc (intermediates, deleted after a successful build unless
      --keep is given) and compile
      ref_hlsl_harness.cpp, which includes them together with hlsl_shim.hpp, into oracle/_ref/libref_hlsl.so.
-The GPU box has no /root/reference: it uses the prebuilt library that travels with the tree."""
+The tests do not load the library: tests/golden/make_ref_hlsl_golden.py runs it once and stores what it computed
+(tests/golden/ref_hlsl.npz), so the comparison with the reference needs neither its checkout nor this build."""
 from __future__ import annotations
 
 import re
@@ -24,7 +27,6 @@ from pathlib import Path
 
 HERE = Path(__file__).resolve().parent
 OUT = HERE.parent / "_ref"
-REF = Path("/root/reference/package/Shaders")
 
 SEMANTIC = re.compile(r"\s*:\s*(SV_\w+|TEXCOORD\d*|COLOR\d*|POSITION\d*)\b")
 FLOAT_LIT = re.compile(r"(?<![\w.])((?:\d+\.\d*|\.\d+)(?:[eE][+-]?\d+)?|\d+[eE][+-]?\d+)(?![\w.])")
@@ -132,9 +134,14 @@ def slice_compute(text: str, sh_text: str) -> str:
 
 
 def main() -> int:
-    if not REF.exists():
-        print("build_ref_hlsl: %s not present (GPU box?): keeping the prebuilt library" % REF)
-        return 0
+    args = [a for a in sys.argv[1:] if a != "--keep"]
+    if len(args) != 1:
+        sys.stderr.write("usage: build_ref_hlsl.py <reference checkout> [--keep]\n")
+        return 2
+    REF = Path(args[0]) / "package" / "Shaders"
+    if not REF.is_dir():
+        sys.stderr.write("build_ref_hlsl: %s is not a directory\n" % REF)
+        return 1
     OUT.mkdir(exist_ok=True)
     gs = (REF / "GaussianSplatting.hlsl").read_text()
     sh = (REF / "SphericalHarmonics.hlsl").read_text()
