@@ -243,8 +243,6 @@ GS_API int gs_unshuffle_bands(GsContext *ctx, const void *gathered, uint32_t par
  *     (GsRenderOptions.row_begin/row_end), rebalanced every frame from the measured per-row cost, composited straight
  *     into place, then one NCCL exchange of the row ranges (SURVEY 8e.1: "a single all-gather of the composited tile buffers";
  *     grouped broadcasts of the exact sizes, in place, on a transfer stream that overlaps the next frame's sort).
- * Environment switches (diagnostics): GS_GROUP_P2P=0 (NCCL for the order too), GS_GROUP_ORDER_ALLGATHER=0 / GS_GROUP_XFER=sendrecv
- * (exact-size broadcasts / send-recv instead of the all-gather), GS_GROUP_VIEW_LATE=1 (view-calc only under the exchange).
  * Two ways to form a group:
  *   gs_group_join    one process per GPU (torchrun-style): every process passes its own context, the group size, its rank
  *                    and the 128-byte id rank 0 got from gs_group_unique_id (sent over any host channel);
@@ -308,10 +306,6 @@ GS_API int gs_readback_order(GsAsset *asset, uint32_t *dst);      /* _SplatSortK
 GS_API int gs_readback_keys(GsAsset *asset, uint32_t *dst);       /* _SplatSortDistances, N words (sorted after gs_sort) */
 GS_API int gs_readback_view(GsAsset *asset, void *dst);           /* _SplatViewData, N x 40 bytes (S/GaussianSplatting.hlsl:610-615) */
 GS_API int gs_upload_order(GsAsset *asset, const uint32_t *src);  /* seed a previous-frame order */
-
-/* Diagnostics: with GS_RASTER_STATS=1 in the environment the compositor counts, per frame, [0] warp-batches,
- * [1] warp cull ballots, [2] warp candidates, [3] warp evaluations, [4] pixel blends, [5] list entries x warps. */
-GS_API int gs_debug_raster_stats(GsContext *ctx, uint64_t out[8]);
 
 /* ---- Unity render-thread entry (SURVEY 8f N2) -------------------------------------- */
 /* Unity executes native GPU work on its render thread through CommandBuffer.IssuePluginEventAndData(func, eventId, data)

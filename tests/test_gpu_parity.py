@@ -223,39 +223,6 @@ def test_tile_partition_bands_reassemble_the_full_frame(g, O, ctx, count, band):
     r.Dispose()
 
 
-def test_raster_tma_variant_identical(g, O, ctx, tmp_path):
-    """k_raster's cp.async.bulk + mbarrier staging (GS_RASTER_TMA=1, read once per process, hence the child process)
-    produces the same render target bits as the default cp.async staging, including long lists and early-outs."""
-    import os
-    import subprocess
-    import sys
-    from pathlib import Path
-    root = Path(__file__).resolve().parents[1]
-    script = (
-        "import sys, numpy as np\n"
-        "sys.path.insert(0, %r); sys.path.insert(0, %r)\n"
-        "import unitygaussiansplatting_b200 as g\n"
-        "from util import camera\n"
-        "ctx = g.GaussianSplatContext(0)\n"
-        "out = {}\n"
-        "for name, n, w, h, q in (('a', 50000, 400, 300, 'Medium'), ('b', 200000, 333, 211, 'VeryHigh')):\n"
-        "    asset = g.synthetic_asset(g.SCENE_CLUSTERED, n, 0x5EED0011, q)\n"
-        "    r = g.GaussianSplatRenderer(asset, ctx)\n"
-        "    rt = np.zeros((h, w, 4), np.float16)\n"
-        "    r.SortAndRenderSplats(camera(g, w, h), rt=rt)\n"
-        "    out[name] = rt\n"
-        "np.savez(sys.argv[1], **out)\n" % (str(root), str(root / "tests")))
-    res = {}
-    for flag in ("0", "1"):
-        path = tmp_path / ("rt%s.npz" % flag)
-        env = dict(os.environ, GS_RASTER_TMA=flag)
-        subprocess.run([sys.executable, "-c", script, str(path)], check=True, env=env, timeout=300)
-        res[flag] = np.load(path)
-    for k in ("a", "b"):
-        assert res["0"][k].any()
-        assert np.array_equal(res["0"][k].view(np.uint16), res["1"][k].view(np.uint16))
-
-
 def test_async_readback_equals_blocking(g, ctx):
     """GS_FLAG_ASYNC_READBACK: host images are filled by a copy stream while the next frame runs; after gs_sync they hold
     exactly what the blocking path returns, for several frames in rotation over two pinned images."""

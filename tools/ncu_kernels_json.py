@@ -28,9 +28,9 @@ def main():
             continue
         full = d[col["Kernel Name"]].split("(")[0].replace("void ", "").replace("gs::", "")
         name = full.split("<")[0]
-        if name == "k_onesweep" and "<" in full:   # <BITS, GATHER, THREADS, PERSIST, KPT>: the persistent variant is the bin sort, not the depth sort
+        if name == "k_onesweep" and "<" in full:   # <BITS, GATHER, PERSIST>: the persistent variant is the bin sort, not the depth sort
             targs = [a.strip() for a in full[full.index("<") + 1:full.rindex(">")].split(",")]
-            if len(targs) >= 4 and targs[3] in ("1", "true", "(bool)1"):
+            if len(targs) >= 3 and targs[2] in ("1", "true", "(bool)1"):
                 name = "k_onesweep_binsort"
         a = acc[name]
 

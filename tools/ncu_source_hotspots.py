@@ -10,7 +10,7 @@ import io
 import subprocess
 import sys
 
-KERNELS = [("k_onesweep (the first one captured: <8, no gather, 256, one-shot, 16>, a depth-sort pass)", "regex:k_onesweep"),
+KERNELS = [("k_onesweep (the first one captured: <8, no gather, one-shot>, a depth-sort pass)", "regex:k_onesweep"),
            ("k_raster (default instantiation)", "regex:k_raster"), ("k_calc_view<Norm6 SH, fused cull>", "regex:k_calc_view"),
            ("k_bin_emit", "regex:k_bin_emit"), ("k_calc_distances", "regex:k_calc_distances")]
 TOP = 12

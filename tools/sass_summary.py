@@ -13,12 +13,11 @@ from pathlib import Path
 
 ROOT = Path(__file__).resolve().parents[1]
 LIB = ROOT / "unitygaussiansplatting_b200" / "libgsplat_b200.so"
-WANT = [("k_onesweep<8, gather, 256, one-shot, 16 keys/thread> (depth sort pass 0)", r"k_onesweepILi8ELb1ELi256ELb0ELi16E"),
-        ("k_onesweep<8, no gather, 256, one-shot, 16> (depth sort passes 1-3, slab sorts)", r"k_onesweepILi8ELb0ELi256ELb0ELi16E"),
-        ("k_onesweep<8, no gather, 256, persistent, 16> (the bin sort)", r"k_onesweepILi8ELb0ELi256ELb1ELi16E"),
-        ("k_raster<fp16 ROP, RGBA16F, no stats, cp.async staging, no extras> (default)", r"k_rasterILb1ELi0ELb0ELb0ELb0E"),
-        ("k_raster<fp16 ROP, RGBA16F, no stats, cp.async.bulk + mbarrier staging, no extras>", r"k_rasterILb1ELi0ELb0ELb1ELb0E"),
-        ("k_raster<fp16 ROP, RGBA16F, no stats, cp.async, EXTRAS> (selected splats / scene depth test)", r"k_rasterILb1ELi0ELb0ELb0ELb1E"),
+WANT = [("k_onesweep<8, gather, one-shot> (depth sort pass 0)", r"k_onesweepILi8ELb1ELb0E"),
+        ("k_onesweep<8, no gather, one-shot> (depth sort passes 1-3, slab sorts)", r"k_onesweepILi8ELb0ELb0E"),
+        ("k_onesweep<8, no gather, persistent> (the bin sort)", r"k_onesweepILi8ELb0ELb1E"),
+        ("k_raster<fp16 ROP, RGBA16F, no extras> (default)", r"k_rasterILb1ELi0ELb0E"),
+        ("k_raster<fp16 ROP, RGBA16F, EXTRAS> (selected splats / scene depth test)", r"k_rasterILb1ELi0ELb1E"),
         ("k_calc_view<3, true, false> (Norm6 SH, fused cull: the Medium frame)", r"k_calc_viewILi3ELb1ELb0E"),
         ("k_calc_distances<0>", r"k_calc_distancesILi0E"), ("k_calc_distances<3> (group of 4: slab table)", r"k_calc_distancesILi3E"),
         ("k_compact_order", r"k_compact_order"), ("k_bin_emit", r"k_bin_emit"), ("k_push_slab (peer stores over NVLink)", r"k_push_slab"),

@@ -143,7 +143,6 @@ NATIVE_SYMBOLS = {
     "gs_unity_get_render_event_func": (GsUnityRenderEventAndDataFunc, []),
     "gs_unity_frame_event_size": (C.c_uint32, []),
     "gs_export_splats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p]),
-    "gs_debug_raster_stats": (C.c_int, [C.c_void_p, C.c_void_p]),
     "gs_context_stream": (C.c_void_p, [C.c_void_p]),
     "gs_asset_device_ptr": (C.c_void_p, [C.c_void_p, C.c_int]),
 }

@@ -121,7 +121,6 @@ int ensure_sort_scratch(GsContext *ctx, uint32_t capacity) {
   ctx->lookback_words = sort_lookback_words(capacity, 4);
   GS_CUDA_TRY(ctx, cudaMalloc(&ctx->sort.lookback, ctx->lookback_words * 4));
   ctx->sort.max_tiles = (capacity + kSortTileItems - 1) / kSortTileItems;
-  ctx->sort.lookback_words = ctx->lookback_words;
   ctx->sort_capacity = capacity;
   return GS_OK;
 }
@@ -834,15 +833,6 @@ static void gs_unity_on_render_event(int event_id, void *data) {
 }
 GsUnityRenderEventAndDataFunc gs_unity_get_render_event_func(void) { return gs_unity_on_render_event; }
 uint32_t gs_unity_frame_event_size(void) { return (uint32_t)sizeof(GsUnityFrameEvent); }
-
-int gs_debug_raster_stats(GsContext *ctx, uint64_t out[8]) {
-  if (!ctx || !out) return GS_ERR_INVALID_ARGUMENT;
-  memset(out, 0, 64);
-  if (!g_raster_stats) return GS_ERR_NOT_READY;
-  GS_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-  GS_CUDA_TRY(ctx, cudaMemcpy(out, g_raster_stats, 64, cudaMemcpyDeviceToHost));
-  return GS_OK;
-}
 
 void *gs_context_stream(GsContext *ctx) { return ctx ? (void *)ctx->stream : nullptr; }
 void *gs_asset_device_ptr(GsAsset *as, int which) {

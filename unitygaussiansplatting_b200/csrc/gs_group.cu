@@ -23,7 +23,6 @@
 // place.  Row exchange: grouped NCCL broadcasts in place.  In GS_GROUP_EMULATE, or without NCCL in a single process, plain
 // device-to-device copies ordered by events stand in for every exchange.
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <new>
 #include <vector>
@@ -81,7 +80,6 @@ struct GsGroup {
   uint32_t size = 0;
   std::vector<Member> m;
   bool emulate = false, use_nccl = false;
-  int xfer = 0;   // 0: grouped broadcasts, 1: grouped send/recv  (GS_GROUP_XFER=bcast|sendrecv)
   uint64_t frame = 0;
   uint32_t hist_w = 0, hist_h = 0;
   uint64_t hist_frames = 0;   // frames rendered at (hist_w, hist_h): the cost of frame k is usable from frame k+2 on
@@ -186,16 +184,8 @@ int exchange_add(GsGroup *g, uint8_t *const *bufs, const size_t *off, const size
     const NcclApi &nc = nccl_api();
     for (size_t i = 0; i < g->m.size(); ++i) {
       Member &mb = g->m[i];
-      if (g->xfer == 1) {
-        for (uint32_t p = 0; p < G; ++p) {
-          if (p == mb.rank) continue;
-          if (cnt[mb.rank]) GS_NCCL_TRY_G(mb.ctx, nc.Send(bufs[i] + off[mb.rank], cnt[mb.rank], ncclUint8, (int)p, mb.comm, st(mb)));
-          if (cnt[p]) GS_NCCL_TRY_G(mb.ctx, nc.Recv(bufs[i] + off[p], cnt[p], ncclUint8, (int)p, mb.comm, st(mb)));
-        }
-      } else {
-        for (uint32_t c = 0; c < G; ++c)
-          if (cnt[c]) GS_NCCL_TRY_G(mb.ctx, nc.Broadcast(bufs[i] + off[c], bufs[i] + off[c], cnt[c], ncclUint8, (int)c, mb.comm, st(mb)));
-      }
+      for (uint32_t c = 0; c < G; ++c)
+        if (cnt[c]) GS_NCCL_TRY_G(mb.ctx, nc.Broadcast(bufs[i] + off[c], bufs[i] + off[c], cnt[c], ncclUint8, (int)c, mb.comm, st(mb)));
     }
     return GS_OK;
   }
@@ -401,12 +391,6 @@ int gs_group_unique_id(void *id_out) {
   return GS_OK;
 }
 
-static int group_env(GsGroup *g) {
-  const char *x = getenv("GS_GROUP_XFER");
-  g->xfer = (x && !strcmp(x, "sendrecv")) ? 1 : 0;
-  return GS_OK;
-}
-
 int gs_group_join(GsContext *ctx, uint32_t group_size, uint32_t rank, const void *id, GsGroup **out) {
   if (!ctx || !out || !id || group_size == 0 || group_size > GS_GROUP_MAX_GPUS || rank >= group_size)
     return fail(ctx, GS_ERR_INVALID_ARGUMENT, "bad group size / rank / id");
@@ -416,7 +400,6 @@ int gs_group_join(GsContext *ctx, uint32_t group_size, uint32_t rank, const void
   if (!g) return fail(ctx, GS_ERR_OUT_OF_MEMORY, "host allocation failed");
   g->size = group_size;
   g->use_nccl = true;
-  group_env(g);
   g->m.resize(1);
   g->m[0].ctx = ctx;
   g->m[0].rank = rank;
@@ -443,7 +426,6 @@ int gs_group_create(const int *devices, uint32_t n, uint32_t flags, GsGroup **ou
   if (!g) return fail(nullptr, GS_ERR_OUT_OF_MEMORY, "host allocation failed");
   g->size = n;
   g->emulate = (flags & GS_GROUP_EMULATE) != 0;
-  group_env(g);
   g->m.resize(n);
   int rc = GS_OK;
   for (uint32_t i = 0; i < n && rc == GS_OK; ++i) {
@@ -456,8 +438,7 @@ int gs_group_create(const int *devices, uint32_t n, uint32_t flags, GsGroup **ou
     rc = member_init(g->m[i]);
   }
   if (rc == GS_OK && !g->emulate && n > 1) {
-    const char *force = getenv("GS_GROUP_NO_NCCL");
-    if (nccl_api().ok() && !(force && force[0] == '1')) {
+    if (nccl_api().ok()) {
       std::vector<ncclComm_t> comms(n);
       ncclResult_t r = nccl_api().CommInitAll(comms.data(), (int)n, devices);
       if (r != ncclSuccess) rc = fail_nccl(nullptr, r, "ncclCommInitAll");
@@ -560,28 +541,6 @@ int gs_group_frame(GsGroup *g, GsAsset *const *assets, const GsFrameParams *fp, 
 
   const bool timing = g->m[0].ctx->timing;
   g->timed = timing;
-  // View-calc reads nothing the sort writes: it runs on the helper stream (lowest priority).  By default it starts with the
-  // frame and fills whatever the sort chain leaves idle (the host wait for the slab table, kernel tails, the exchange);
-  // GS_GROUP_VIEW_LATE=1 starts it only when the slab sort is done, i.e. squarely under the order exchange.
-  static int view_late_env = -1;
-  if (view_late_env < 0) { const char *e = getenv("GS_GROUP_VIEW_LATE"); view_late_env = (e && e[0] == '1') ? 1 : 0; }
-  const bool view_late = view_late_env && do_sort_flag && G > 1;
-  auto enqueue_view = [&](size_t i, cudaEvent_t after) -> int {
-    Member &mb = g->m[i];
-    GsContext *ctx = mb.ctx;
-    GsRenderOptions opt = base;
-    opt.row_begin = g->bounds[mb.rank]; opt.row_end = g->bounds[mb.rank + 1];
-    if (opt.row_end > opt.row_begin || G == 1) {
-      if (G == 1) opt.row_begin = opt.row_end = 0;
-      GS_CUDA_TRY(ctx, cudaStreamWaitEvent(mb.aux, after, 0));
-      if (timing) cudaEventRecord(mb.tev[GT_V0], mb.aux);
-      int r = do_view(ctx, assets[i], fp, fc, true, opt, mb.aux);
-      if (r) return r;
-      if (timing) cudaEventRecord(mb.tev[GT_V1], mb.aux);
-      GS_CUDA_TRY(ctx, cudaEventRecord(mb.ev_view, mb.aux));
-    }
-    return GS_OK;
-  };
   GsNvtxRange nvtx_frame("GaussianSplat.GroupFrame");
   // ---- phase A: distances + slab table on the context stream; view-calc on the second stream --------------------------
   for (size_t i = 0; i < L; ++i) {
@@ -608,12 +567,20 @@ int gs_group_frame(GsGroup *g, GsAsset *const *assets, const GsFrameParams *fp, 
       }
     }
     if (timing) cudaEventRecord(mb.tev[GT_DIST], ctx->stream);
-    // view-calc starts right behind the distance kernel (started together, its 24 k blocks crowd the distance kernel out:
-    // 63 instead of 32 us at N = 8) and so runs under the host's wait for the slab table, the sort's tails and the exchange
-    if (!view_late) {
-      cudaEvent_t after = mb.ev_begin;
-      if (do_sort_flag) { GS_CUDA_TRY(ctx, cudaEventRecord(mb.ev_produced, ctx->stream)); after = mb.ev_produced; }
-      if ((rc = enqueue_view(i, after))) return rc;
+    // View-calc reads nothing the sort writes: it runs on the helper stream (lowest priority), right behind the distance
+    // kernel (started together, its 24 k blocks crowd the distance kernel out: 63 instead of 32 us at N = 8), and fills
+    // whatever the sort chain leaves idle: the host's wait for the slab table, the sort's tails and the exchange
+    cudaEvent_t after = mb.ev_begin;
+    if (do_sort_flag) { GS_CUDA_TRY(ctx, cudaEventRecord(mb.ev_produced, ctx->stream)); after = mb.ev_produced; }
+    GsRenderOptions opt = base;
+    opt.row_begin = g->bounds[mb.rank]; opt.row_end = g->bounds[mb.rank + 1];
+    if (opt.row_end > opt.row_begin || G == 1) {
+      if (G == 1) opt.row_begin = opt.row_end = 0;
+      GS_CUDA_TRY(ctx, cudaStreamWaitEvent(mb.aux, after, 0));
+      if (timing) cudaEventRecord(mb.tev[GT_V0], mb.aux);
+      if ((rc = do_view(ctx, as, fp, fc, true, opt, mb.aux))) return rc;
+      if (timing) cudaEventRecord(mb.tev[GT_V1], mb.aux);
+      GS_CUDA_TRY(ctx, cudaEventRecord(mb.ev_view, mb.aux));
     }
   }
 
@@ -645,12 +612,8 @@ int gs_group_frame(GsGroup *g, GsAsset *const *assets, const GsFrameParams *fp, 
     uint32_t cap = 0;
     for (uint32_t c = 0; c < G; ++c) cap = g->slab_cnt[c] > cap ? g->slab_cnt[c] : cap;
     cap = (cap + 3u) & ~3u;
-    static int ag_env = -1;
-    if (ag_env < 0) { const char *e = getenv("GS_GROUP_ORDER_ALLGATHER"); ag_env = (e && e[0] == '0') ? 0 : 1; }
-    // one process per GPU: slabs go peer to peer (set up on the first sorted frame; GS_GROUP_P2P=0 keeps NCCL)
-    static int p2p_env = -1;
-    if (p2p_env < 0) { const char *e = getenv("GS_GROUP_P2P"); p2p_env = (e && e[0] == '0') ? 0 : 1; }
-    if (G > 1 && g->use_nccl && L == 1 && p2p_env && !g->link.tried) { if ((rc = peer_link_setup(g, assets[0]))) return rc; }
+    // one process per GPU: slabs go peer to peer (set up on the first sorted frame)
+    if (G > 1 && g->use_nccl && L == 1 && !g->link.tried) { if ((rc = peer_link_setup(g, assets[0]))) return rc; }
     const bool use_p2p = G > 1 && L == 1 && g->link.ready && g->link.asset == assets[0];
     uint32_t *p2p_new = nullptr;
     int p2p_idx = 0;
@@ -658,7 +621,7 @@ int gs_group_frame(GsGroup *g, GsAsset *const *assets, const GsFrameParams *fp, 
       p2p_idx = assets[0]->order == g->link.buf[0] ? 1 : 0;
       p2p_new = g->link.buf[p2p_idx];
     }
-    const bool use_gather = !use_p2p && G > 1 && ag_env && g->xfer == 0 && (uint64_t)cap * G <= (uint64_t)N + (uint64_t)N / 2 + 64u * G;
+    const bool use_gather = !use_p2p && G > 1 && (uint64_t)cap * G <= (uint64_t)N + (uint64_t)N / 2 + 64u * G;
     if (use_gather) {
       for (size_t i = 0; i < L; ++i) {
         Member &mb = g->m[i];
@@ -706,10 +669,6 @@ int gs_group_frame(GsGroup *g, GsAsset *const *assets, const GsFrameParams *fp, 
       }
       GS_CUDA_TRY(ctx, cudaGetLastError());
       if (timing) cudaEventRecord(mb.tev[GT_SORT], ctx->stream);
-      if (view_late) {
-        GS_CUDA_TRY(ctx, cudaEventRecord(mb.ev_produced, ctx->stream));   // (free until the exchange records it again)
-        if ((rc = enqueue_view(i, mb.ev_produced))) return rc;
-      }
     }
     if (G > 1) {
       std::vector<uint8_t *> bufs(L);

@@ -143,7 +143,6 @@ struct SortScratch {
   uint32_t *lookback;             // passes * max_tiles * 256 status words
   uint32_t *tickets;              // passes counters
   uint32_t max_tiles;             // capacity / kSortTileItems rounded up
-  size_t lookback_words;          // size of `lookback`
 };
 constexpr uint32_t kSortTileItems = 4096;  // 256 threads x 16 keys
 size_t sort_lookback_words(uint32_t capacity, int passes);
@@ -178,7 +177,6 @@ BinScratch launch_binning(const FrameConsts &fc, const GsRenderOptions &opt, uin
 // zndc / scene_depth: per-splat quad depth and the W x H depth buffer to test it against (both nullptr: no depth test)
 void launch_raster(const FrameConsts &fc, const GsRenderOptions &opt, const float4 *draw, const BinScratch &bs, void *rt,
                    uint32_t rt_pitch_bytes, uint32_t rt_format, cudaStream_t s, const float *zndc = nullptr, const float *scene_depth = nullptr);
-extern unsigned long long *g_raster_stats;   // diagnostics, see GS_RASTER_STATS
 uint32_t partition_own_bin_rows(const GsRenderOptions &opt, uint32_t binsY);
 uint32_t partition_own_tile_rows(const GsRenderOptions &opt, uint32_t binsY);
 void launch_unshuffle(const void *gathered, uint32_t parts, uint32_t band, uint32_t rows_pp, uint32_t fmt, void *out, uint32_t pitch,

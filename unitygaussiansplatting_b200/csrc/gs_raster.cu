@@ -318,60 +318,22 @@ void launch_row_costs(const uint32_t *cost, uint32_t ntx, uint32_t t0, uint32_t 
   if (t1 > t0) k_row_costs<<<(t1 - t0 + 7) / 8, 256, 0, s>>>(cost, ntx, t0, t1, row_cost);
 }
 
-// ---- TMA (bulk async copy) staging: one 48-byte cp.async.bulk per record, completion counted in bytes on an mbarrier ----
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t *bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t *bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "GS_WAIT:\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-      "@p bra GS_DONE;\n\t"
-      "bra GS_WAIT;\n\t"
-      "GS_DONE:\n\t}" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void bulk_copy_g2s(void *smem_dst, const void *gmem_src, uint32_t bytes, uint64_t *bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(smem_dst)),
-               "l"(gmem_src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}
-
 // SEL ("extras"): a separate instantiation for frames with an edit selection and / or a scene depth buffer bound, so that
 // ordinary frames pay nothing.  Selected splats (records with opacity -1) take the pixel shader's other branch
 // (S/RenderGaussianSplats.shader:87-101); with `scene_depth` every fragment is depth-tested like the pass's ZTest LEqual
 // (reversed Z: quad depth >= stored depth), the per-splat quad depths being staged beside the records.
-template <bool FP16_ROP, int OUT_FMT, bool STATS, bool TMA, bool SEL = false>
+template <bool FP16_ROP, int OUT_FMT, bool SEL>
 __global__ void __launch_bounds__(256)
 k_raster(FrameConsts fc, Partition part, const float4 *__restrict__ draw, const uint2 *__restrict__ bin_ranges,
          const uint32_t *__restrict__ tile_vals, const uint32_t *__restrict__ tile_order, uint32_t *__restrict__ tile_cost, uint32_t ntx,
-         uint8_t *__restrict__ rt, uint32_t pitch, uint32_t band_packed, uint32_t load_rt, unsigned long long *stats,
+         uint8_t *__restrict__ rt, uint32_t pitch, uint32_t band_packed, uint32_t load_rt,
          const float *__restrict__ zndc, const float *__restrict__ scene_depth) {
-  uint32_t st_batches = 0, st_culls = 0, st_cand = 0, st_eval = 0, st_blend = 0;   // GS_RASTER_STATS diagnostics (per warp)
-  unsigned long long st_t0 = 0;
-  if (STATS) asm volatile("mov.u64 %0, %globaltimer;" : "=l"(st_t0));
-  // two staging buffers of 256 raster records (3 x float4 each): batch k+1 lands asynchronously while batch k is composited.
-  // cp.async path: planar [buf][plane][entry]; TMA path: the 48-byte records as they are, [buf][entry][plane].
+  uint32_t st_batches = 0, st_eval = 0;   // this warp's work, for the tile's cost below
+  // two staging buffers of 256 raster records (3 x float4 each), planar [buf][plane][entry]: batch k+1 lands asynchronously
+  // while batch k is composited
   __shared__ __align__(128) float4 s_rec[2][3][256];  // plane 0: cx, cy, i1x, i1y   1: i2x, i2y, opacity, hx   2: r, g, b, hy
-  __shared__ __align__(8) uint64_t s_bar[2];
   __shared__ float s_z[SEL ? 2 : 1][SEL ? 256 : 1];   // quad depths of the staged batch (depth test only)
   const bool depth_test = SEL && scene_depth != nullptr;
-  constexpr int ES = TMA ? 3 : 1;     // float4 stride between consecutive entries of one plane
-  constexpr int PS = TMA ? 1 : 256;   // float4 stride between the planes of one entry
-  if (TMA) {
-    if (threadIdx.x == 0) {
-      mbar_init(&s_bar[0], 256);
-      mbar_init(&s_bar[1], 256);
-      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-  }
 
   const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   // 1-D grid over raster tiles: tile = (16-pixel column, R * own 64-pixel bin row + tile row inside that bin row)
@@ -414,17 +376,6 @@ k_raster(FrameConsts fc, Partition part, const float4 *__restrict__ draw, const 
   // three-deep pipeline: splat ids of batch k+2 (register) -> records of batch k+1 (cp.async in flight) -> batch k (composited)
   auto load_id = [&](uint32_t e) -> uint32_t { return e < range.y ? __ldg(tile_vals + e) : 0xFFFFFFFFu; };
   auto stage = [&](int buf, uint32_t id) {
-    float4 *base_f4 = &s_rec[buf][0][0];
-    if (TMA) {
-      // every thread arrives once per stage; a thread with a record first announces its 48 bytes, then issues the bulk copy
-      if (id != 0xFFFFFFFFu) {
-        mbar_arrive_expect_tx(&s_bar[buf], 48u);
-        bulk_copy_g2s(base_f4 + (size_t)tid * 3, draw + (size_t)id * 3, 48u, &s_bar[buf]);
-      } else {
-        mbar_arrive(&s_bar[buf]);
-      }
-      return;
-    }
     if (id != 0xFFFFFFFFu) {
       const float4 *src = draw + (size_t)id * 3;
       cp_async16(&s_rec[buf][0][tid], src);
@@ -436,42 +387,34 @@ k_raster(FrameConsts fc, Partition part, const float4 *__restrict__ draw, const 
   };
   uint32_t id_next = load_id(range.x + tid);
   stage(0, id_next);
-  uint32_t issued = 0;   // index of the newest stage handed to the copy engine
   id_next = load_id(range.x + 256 + tid);
 
   int buf = 0;
-  uint32_t kbatch = 0;   // stage index: stage s lives in buffer s&1 and completes phase (s>>1)&1 of that buffer's mbarrier
-  for (uint32_t base = range.x; base < range.y; base += 256, buf ^= 1, ++kbatch) {
-    stage(buf ^ 1, id_next); issued = kbatch + 1;  // batch k+1 -> other buffer (free since the barrier that ended batch k-1)
-    id_next = load_id(base + 512 + tid);           // ids of batch k+2
-    if (TMA) {
-      mbar_wait(&s_bar[buf], (kbatch >> 1) & 1u);  // all 256 arrivals + every announced byte of batch k have landed
-    } else {
-      cp_async_wait<1>();                          // batch k has landed (this thread's copies) ...
-      __syncthreads();                             // ... and everyone else's
-    }
-    const float4 *s_a = &s_rec[buf][0][0], *s_b = s_a + PS, *s_c = s_a + 2 * PS;
+  for (uint32_t base = range.x; base < range.y; base += 256, buf ^= 1) {
+    stage(buf ^ 1, id_next);              // batch k+1 -> other buffer (free since the barrier that ended batch k-1)
+    id_next = load_id(base + 512 + tid);  // ids of batch k+2
+    cp_async_wait<1>();                   // batch k has landed (this thread's copies) ...
+    __syncthreads();                      // ... and everyone else's
+    const float4 *s_a = s_rec[buf][0], *s_b = s_rec[buf][1], *s_c = s_rec[buf][2];
 
     const uint32_t cnt = min(256u, range.y - base);
     ++st_batches;
     for (uint32_t c0 = 0; c0 < cnt; c0 += 32) {
       // a warp whose 32 pixels all reached dst.a == 1 ignores everything behind exactly: skip the batch remainder
       if (__all_sync(0xffffffffu, d3 == 1.0f || !in_image)) break;
-      if (STATS) ++st_culls;
       // one ballot culls 32 splats against this warp's 8x4 pixel block
       const uint32_t e = c0 + lane;
       bool hit = false;
       if (e < cnt) {
-        const float4 A = s_a[e * ES];
-        const float hx = s_b[e * ES].w, hy = s_c[e * ES].w;
+        const float4 A = s_a[e];
+        const float hx = s_b[e].w, hy = s_c[e].w;
         hit = (fabsf(A.x - bcx) <= hx + 3.5f) && (fabsf(A.y - bcy) <= hy + 1.5f);
       }
       uint32_t mask = __ballot_sync(0xffffffffu, hit);
       while (mask) {
         const uint32_t j = c0 + __ffs(mask) - 1;
         mask &= mask - 1;
-        if (STATS) ++st_cand;
-        const float4 A = s_a[j * ES], B = s_b[j * ES];
+        const float4 A = s_a[j], B = s_b[j];
         const float dx = pxc - A.x, dy = A.y - pyc;  // pixel y grows down, NDC y up
         const float qa = fmaf(dy, A.w, dx * A.z), qb = fmaf(dy, B.y, dx * B.x);
         const bool inside = (fabsf(qa) <= 2.0f) && (fabsf(qb) <= 2.0f);  // quad corners at +-2 (:54-55)
@@ -492,8 +435,7 @@ k_raster(FrameConsts fc, Partition part, const float4 *__restrict__ draw, const 
         bool pass = inside && alpha >= 0.003921569f;                      // discard below 1/255 (:103-104)
         if (SEL && depth_test) pass = pass && (s_z[SEL ? buf : 0][SEL ? j : 0] >= zscene);   // ZTest LEqual, reversed Z
         if (pass) {
-          if (STATS) ++st_blend;
-          float4 C = s_c[j * ES];
+          float4 C = s_c[j];
           if (SEL && tint) {
             if (outline) { C.x = 1.0f; C.y = 0.0f; C.z = 1.0f; }
             C.x = lerpf(C.x, 1.0f, 0.5f); C.y = lerpf(C.y, 0.0f, 0.5f); C.z = lerpf(C.z, 1.0f, 0.5f);
@@ -513,29 +455,11 @@ k_raster(FrameConsts fc, Partition part, const float4 *__restrict__ draw, const 
     // frees this batch's buffer for the copies issued at the top of the next-but-one iteration.
     if (__syncthreads_and(d3 == 1.0f || !in_image)) break;
   }
-  if (TMA) {
-    // exactly one issued stage has not been waited for (the look-ahead one, or stage 0 of an empty list): drain it
-    mbar_wait(&s_bar[issued & 1u], (issued >> 1) & 1u);
-  } else {
-    cp_async_wait<0>();
-  }
+  cp_async_wait<0>();
   // this tile's cost for next frame's launch order: the slowest warp's work (evaluations dominate, culls and batches add)
   if (lane == 0) atomicMax(&s_cost, st_eval * 4 + st_batches * 16 + 1);
   __syncthreads();
   if (threadIdx.x == 0) tile_cost[lin] = s_cost;
-  if (STATS) {
-    const uint32_t bl = __reduce_add_sync(0xffffffffu, st_blend);
-    if (lane == 0) {
-      atomicAdd(stats + 0, (unsigned long long)st_batches); atomicAdd(stats + 1, (unsigned long long)st_culls);
-      atomicAdd(stats + 2, (unsigned long long)st_cand); atomicAdd(stats + 3, (unsigned long long)st_eval);
-      atomicAdd(stats + 4, (unsigned long long)bl); atomicAdd(stats + 5, (unsigned long long)(range.y - range.x));
-      unsigned long long t1;
-      asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t1));
-      atomicAdd(stats + 6, t1 - st_t0);
-      atomicMax(stats + 7, t1 - st_t0);
-    }
-  }
-
   if (in_image) {
     uint8_t *row = rt + (size_t)out_row * pitch;
     if (OUT_FMT == GS_PIX_RGBA16F) {
@@ -549,9 +473,6 @@ k_raster(FrameConsts fc, Partition part, const float4 *__restrict__ draw, const 
   }
 }
 
-unsigned long long *g_raster_stats = nullptr;
-static constexpr int kRasterTmaDefault = 0;
-
 void launch_raster(const FrameConsts &fc, const GsRenderOptions &opt, const float4 *draw, const BinScratch &bs, void *rt,
                    uint32_t rt_pitch_bytes, uint32_t rt_format, cudaStream_t s, const float *zndc, const float *scene_depth) {
   const Partition part = make_partition(opt);
@@ -562,25 +483,14 @@ void launch_raster(const FrameConsts &fc, const GsRenderOptions &opt, const floa
   k_tile_order<<<1, 1024, 0, s>>>(bs.tile_cost, ntiles, ntx, part, bs.tile_order);
   const bool rop = opt.blend_mode == GS_BLEND_FP16_ROP;
   uint8_t *out = reinterpret_cast<uint8_t *>(rt);
-  // GS_RASTER_STATS=1: per-frame work counters (diagnostics; printed by tools/raster_stats.py through gs_debug_raster_stats)
-  static unsigned long long *stats = nullptr;
-  static int want = -1;
-  if (want < 0) { const char *e = getenv("GS_RASTER_STATS"); want = (e && e[0] == '1') ? 1 : 0; }
-  if (want && !stats) { cudaMalloc(&stats, 64); g_raster_stats = stats; }
-  if (stats) cudaMemsetAsync(stats, 0, 64, s);
-  // GS_RASTER_TMA=0/1: record staging by per-thread cp.async (16 B x 3) or by cp.async.bulk + mbarrier (48 B x 1)
-  static int tma = -1;
-  if (tma < 0) { const char *e = getenv("GS_RASTER_TMA"); tma = e ? (e[0] == '1') : kRasterTmaDefault; }
   const uint32_t bins = fc.binsX * fc.binsY;
   uint2 *ranges = reinterpret_cast<uint2 *>(bs.bin_ranges);
   const uint32_t packed = part.range ? 0u : opt.band_packed, load = (opt.flags & GS_FLAG_LOAD_RT) ? 1u : 0u;
   k_bin_ranges<<<(bins + 7) / 8, 256, 0, s>>>(bs.tile_keys, bs.entry_count, bins, ranges);
 #define GS_LAUNCH_RASTER(ROP, FMT)                                                                                              \
   do {                                                                                                                         \
-    if (fc.selValid || scene_depth) k_raster<ROP, FMT, false, false, true><<<grid, 256, 0, s>>>(fc, part, draw, ranges, bs.tile_vals, bs.tile_order, bs.tile_cost, ntx, out, rt_pitch_bytes, packed, load, stats, zndc, scene_depth); \
-    else if (tma) k_raster<ROP, FMT, false, true><<<grid, 256, 0, s>>>(fc, part, draw, ranges, bs.tile_vals, bs.tile_order, bs.tile_cost, ntx, out, rt_pitch_bytes, packed, load, stats, nullptr, nullptr); \
-    else if (stats) k_raster<ROP, FMT, true, false><<<grid, 256, 0, s>>>(fc, part, draw, ranges, bs.tile_vals, bs.tile_order, bs.tile_cost, ntx, out, rt_pitch_bytes, packed, load, stats, nullptr, nullptr); \
-    else k_raster<ROP, FMT, false, false><<<grid, 256, 0, s>>>(fc, part, draw, ranges, bs.tile_vals, bs.tile_order, bs.tile_cost, ntx, out, rt_pitch_bytes, packed, load, stats, nullptr, nullptr); \
+    if (fc.selValid || scene_depth) k_raster<ROP, FMT, true><<<grid, 256, 0, s>>>(fc, part, draw, ranges, bs.tile_vals, bs.tile_order, bs.tile_cost, ntx, out, rt_pitch_bytes, packed, load, zndc, scene_depth); \
+    else k_raster<ROP, FMT, false><<<grid, 256, 0, s>>>(fc, part, draw, ranges, bs.tile_vals, bs.tile_order, bs.tile_cost, ntx, out, rt_pitch_bytes, packed, load, nullptr, nullptr); \
   } while (0)
   if (rt_format == GS_PIX_RGBA16F) {
     if (rop) GS_LAUNCH_RASTER(true, GS_PIX_RGBA16F); else GS_LAUNCH_RASTER(false, GS_PIX_RGBA16F);

@@ -21,7 +21,6 @@
 // The digit width is a template parameter: depth keys use 4 x 8 bits, the tile binner sorts
 // 12..16-bit tile ids in 2 passes of 6..8 bits.
 // No tensor-core path: there is no contraction here, only byte/integer traffic.
-#include <cstdio>
 #include <cstdlib>
 
 #include "gs_kernels.cuh"
@@ -107,24 +106,20 @@ __device__ __forceinline__ uint32_t match_digit(uint32_t d) {
 }
 
 // ---- one digit pass -------------------------------------------------------------------------
-__device__ __forceinline__ uint64_t gtime() { uint64_t t; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t)); return t; }
-#define GS_TRACE(slot) do { if (trace && tid == 0) trace[(size_t)tile * 8 + (slot)] = gtime(); } while (0)
-
 // GATHER: the keys of this pass are keys_src[payload] (pass 0 of the depth sort reads the per-splat key
 // table through last frame's order, S/SplatUtilities.compute:76-81, without a separate gather pass).
 // PERSIST: a fixed grid whose CTAs keep taking tiles until the (device-side) count is exhausted -- for lists whose length
 // the host does not know when it launches (the binner's entry list): no capacity-sized grid of idle CTAs.
-// KPT: keys per thread (a tile is THREADS * KPT pairs): 16 for big sorts; 8 when the whole sort is about one wave of tiles, where a
-// pass costs one tile latency and half-size tiles have a shorter one.
-template <int BITS, bool GATHER, int THREADS, bool PERSIST, int KPT>
-__global__ void __launch_bounds__(THREADS, 1024 / THREADS)
+template <int BITS, bool GATHER, bool PERSIST>
+__global__ void __launch_bounds__(256, 4)
 k_onesweep(const uint32_t *__restrict__ src_k, const uint32_t *__restrict__ src_v, uint32_t *__restrict__ dst_k,
            uint32_t *__restrict__ dst_v, const uint32_t *__restrict__ d_count, int shift, const uint32_t *__restrict__ ghist,
-           volatile uint32_t *lookback, uint32_t *ticket, uint64_t *trace) {
+           volatile uint32_t *lookback, uint32_t *ticket) {
   constexpr uint32_t NB = 1u << BITS;
-  constexpr uint32_t kTileItems = THREADS * KPT;
-  constexpr int kSortWarps = THREADS / 32;
-  constexpr int kSortThreads = THREADS;
+  constexpr int KPT = 16;   // keys per thread
+  constexpr uint32_t kTileItems = kSortTileItems;   // 256 threads x KPT
+  constexpr int kSortWarps = 8;
+  constexpr int kSortThreads = 256;
   extern __shared__ __align__(16) uint8_t s_dyn[];
   uint2 *s_kv = reinterpret_cast<uint2 *>(s_dyn);                                         // [kTileItems]
   uint32_t (*s_whist)[NB] = reinterpret_cast<uint32_t (*)[NB]>(s_dyn + kTileItems * 8);    // [kSortWarps][NB]
@@ -147,7 +142,6 @@ k_onesweep(const uint32_t *__restrict__ src_k, const uint32_t *__restrict__ src_
   const uint32_t tile = s_tile;
   if (tile >= num_tiles) return;
   const uint32_t tile_base = tile * kTileItems;
-  GS_TRACE(0);
   const bool full_tile = tile_base + kTileItems <= n;
 
   // warp-striped load: warp w owns 512 consecutive pairs, item i of lane l is base + i*32 + l
@@ -184,7 +178,6 @@ k_onesweep(const uint32_t *__restrict__ src_k, const uint32_t *__restrict__ src_
     }
   }
   __syncthreads();
-  GS_TRACE(1);
 
   // 2. publish, then resolve the exclusive prefix over earlier tiles with 4 status probes in flight
   uint32_t prefix = 0, tile_total = 0;
@@ -221,7 +214,6 @@ k_onesweep(const uint32_t *__restrict__ src_k, const uint32_t *__restrict__ src_
     }
   }
   __syncwarp();   // the spin loop above ends per thread: tell the compiler the warp is whole again before the ballots
-  GS_TRACE(2);
   if (!GATHER) {  // payloads: issued now, consumed at the scatter
     if (full_tile) {
 #pragma unroll
@@ -255,7 +247,6 @@ k_onesweep(const uint32_t *__restrict__ src_k, const uint32_t *__restrict__ src_
     __syncwarp();
   }
   __syncthreads();
-  GS_TRACE(3);
 
   // 4. thread `tid` < NB owns digit `tid`: exclusive prefix over warps, tile/global digit bases
   if (tid < NB) {
@@ -274,7 +265,6 @@ k_onesweep(const uint32_t *__restrict__ src_k, const uint32_t *__restrict__ src_
     s_off[tid] = gbase + prefix - dig_start;
   }
   __syncthreads();
-  GS_TRACE(4);
 
   // 5. scatter into digit order inside shared memory
 #pragma unroll
@@ -285,7 +275,6 @@ k_onesweep(const uint32_t *__restrict__ src_k, const uint32_t *__restrict__ src_
     s_kv[pos] = make_uint2(key[i], val[i]);
   }
   __syncthreads();
-  GS_TRACE(5);
 
   const uint32_t valid = full_tile ? kTileItems : n - tile_base;
 #pragma unroll 4
@@ -295,7 +284,6 @@ k_onesweep(const uint32_t *__restrict__ src_k, const uint32_t *__restrict__ src_
     dst_k[dst] = kv.x;
     dst_v[dst] = kv.y;
   }
-  GS_TRACE(6);
   } while (PERSIST);
 }
 
@@ -410,47 +398,19 @@ void launch_compact_order(const uint32_t *order, uint32_t n, const uint32_t *mas
   k_compact_order<<<nblocks, 256, words * 4u, s>>>(order, n, mask, group_bits, words, key_table, out_ids, out_keys, status + 1, status, count_out);
 }
 
-// optional per-tile phase trace of the first pass (debug/profiling aid): GS_SORT_TRACE=<file>
-static uint64_t *g_trace = nullptr;
-static uint32_t g_trace_tiles = 0;
-
-static int sort_threads() {
-  static int v = 0;
-  if (!v) { const char *e = getenv("GS_SORT_THREADS"); v = (e && atoi(e) == 512) ? 512 : 256; }
-  return v;
-}
-
 template <int BITS>
-static void launch_pass(uint32_t count_bound, bool persist, bool small_tiles, cudaStream_t s, const uint32_t *sk, const uint32_t *sv, uint32_t *dk,
+static void launch_pass(uint32_t count_bound, bool persist, cudaStream_t s, const uint32_t *sk, const uint32_t *sv, uint32_t *dk,
                         uint32_t *dv, const uint32_t *d_count, int shift, const uint32_t *ghist, uint32_t *lookback, uint32_t *ticket,
-                        uint64_t *trace, bool gather) {
-  auto go = [&](auto kern, int threads, int kpt) {
-    const size_t smem = (size_t)threads * kpt * 8 + (size_t)(threads / 32) * (1u << BITS) * 4;
-    // the opt-in for > 48 KB dynamic shared memory is per function AND per device
-    struct Seen { const void *fn; int dev; };
-    static thread_local Seen configured[64];
-    static thread_local int nconf = 0;
-    int dev = 0;
-    cudaGetDevice(&dev);
-    bool seen = false;
-    for (int i = 0; i < nconf; ++i) seen |= configured[i].fn == (const void *)kern && configured[i].dev == dev;
-    if (!seen) {
-      cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-      if (nconf < 64) configured[nconf++] = Seen{(const void *)kern, dev};
-    }
-    const uint32_t per = (uint32_t)threads * kpt;
-    uint32_t grid = (uint32_t)(((uint64_t)count_bound + per - 1) / per);
-    if (persist) grid = min(grid, 148u * (1024u / (uint32_t)threads));
-    kern<<<grid, threads, smem, s>>>(sk, sv, dk, dv, d_count, shift, ghist, lookback, ticket, trace);
-  };
+                        bool gather) {
+  // 32 KB of pairs + 8 KB of warp histograms at BITS = 8, plus 3 KB of static shared memory: within the default 48 KB
+  const size_t smem = (size_t)kSortTileItems * 8 + 8 * (1u << BITS) * 4;
+  uint32_t grid = (uint32_t)(((uint64_t)count_bound + kSortTileItems - 1) / kSortTileItems);
+  auto go = [&](auto kern) { kern<<<grid, 256, smem, s>>>(sk, sv, dk, dv, d_count, shift, ghist, lookback, ticket); };
   if (persist) {
-    if (gather) go(k_onesweep<BITS, true, 256, true, 16>, 256, 16); else go(k_onesweep<BITS, false, 256, true, 16>, 256, 16);
-  } else if (small_tiles) {
-    if (gather) go(k_onesweep<BITS, true, 256, false, 8>, 256, 8); else go(k_onesweep<BITS, false, 256, false, 8>, 256, 8);
-  } else if (sort_threads() == 512) {
-    if (gather) go(k_onesweep<BITS, true, 512, false, 16>, 512, 16); else go(k_onesweep<BITS, false, 512, false, 16>, 512, 16);
+    grid = min(grid, 148u * 4u);
+    if (gather) go(k_onesweep<BITS, true, true>); else go(k_onesweep<BITS, false, true>);
   } else {
-    if (gather) go(k_onesweep<BITS, true, 256, false, 16>, 256, 16); else go(k_onesweep<BITS, false, 256, false, 16>, 256, 16);
+    if (gather) go(k_onesweep<BITS, true, false>); else go(k_onesweep<BITS, false, false>);
   }
 }
 
@@ -464,16 +424,10 @@ void launch_sort_pairs(uint32_t *keys, uint32_t *vals, const uint32_t *d_count, 
   // length lives on the device only (the binner's entries): a persistent grid, and the look-back rows actually needed are
   // cleared by a kernel that reads the count.
   const bool persist = !count_is_capacity;
-  // Half-size tiles for exact, smallish counts (a slab of a group's sort) were tried -- twice the CTAs, shorter tiles -- and
-  // measured SLOWER on B200 (24.0 vs 22 us per pass of 1.5 M pairs): a pass is bound by its fixed per-tile work, not by
-  // the tile count.  Kept behind GS_SORT_SMALL_TILES=1 for experiments.
-  static int small_env = -1;
-  if (small_env < 0) { const char *e = getenv("GS_SORT_SMALL_TILES"); small_env = (e && e[0] == '1') ? 1 : 0; }
-  const bool small_tiles = small_env && !persist && capacity <= 4u * 1024u * 1024u && sort_threads() != 512 &&
-                           (size_t)tiles * 2 * nb * passes <= sc.lookback_words;
-  const uint32_t rows = small_tiles ? (capacity + kSortTileItems / 2 - 1) / (kSortTileItems / 2) : tiles;
+  // Half-size tiles for a slab's exact, smallish count were measured slower on B200 (24.0 vs 22 us per pass of 1.5 M pairs):
+  // a pass is bound by its fixed per-tile work, not by the tile count.
   if (persist) k_zero_rows<<<148, 256, 0, s>>>(sc.lookback, d_count, kSortTileItems, nb, nb, (uint32_t)passes, tiles * nb);
-  else cudaMemsetAsync(sc.lookback, 0, (size_t)rows * nb * passes * sizeof(uint32_t), s);
+  else cudaMemsetAsync(sc.lookback, 0, (size_t)tiles * nb * passes * sizeof(uint32_t), s);
   cudaMemsetAsync(sc.tickets, 0, 4 * sizeof(uint32_t), s);
   if (!hist_ready) {
     cudaMemsetAsync(sc.ghist, 0, 4 * 256 * sizeof(uint32_t), s);
@@ -485,36 +439,20 @@ void launch_sort_pairs(uint32_t *keys, uint32_t *vals, const uint32_t *d_count, 
     else k_sort_hist<2, 8><<<grid, 256, 0, s>>>(keys, d_count, sc.ghist);
   }
   uint32_t *sk = keys, *sv = vals, *dk = sc.alt_keys, *dv = sc.alt_vals;
-  const char *trace_path = getenv("GS_SORT_TRACE");
-  if (trace_path && passes == 4 && g_trace_tiles < tiles) {
-    cudaFree(g_trace);
-    cudaMalloc(&g_trace, (size_t)tiles * 8 * sizeof(uint64_t));
-    g_trace_tiles = tiles;
-  }
   for (int p = 0; p < passes; ++p) {
-    uint64_t *trace = (trace_path && passes == 4 && p == 1 && !small_tiles) ? g_trace : nullptr;
-    if (trace) cudaMemsetAsync(trace, 0, (size_t)tiles * 8 * sizeof(uint64_t), s);
     if (pass_events) cudaEventRecord(pass_events[p], s);
-    uint32_t *lb = sc.lookback + (size_t)p * rows * nb;
+    uint32_t *lb = sc.lookback + (size_t)p * tiles * nb;
     const bool gather = key_table != nullptr && p == 0;   // pass 0 reads key_table[vals[i]] instead of keys[i]
     const uint32_t *src_keys = gather ? key_table : sk;
     if (p == passes - 1 && final_keys && final_vals) { dk = final_keys; dv = final_vals; }   // the last pass lands where the caller wants it
-    if (bits == 5) launch_pass<5>(capacity, persist, small_tiles, s, src_keys, sv, dk, dv, d_count, bits * p, sc.ghist + 256 * p, lb, sc.tickets + p, trace, gather);
-    else if (bits == 6) launch_pass<6>(capacity, persist, small_tiles, s, src_keys, sv, dk, dv, d_count, bits * p, sc.ghist + 256 * p, lb, sc.tickets + p, trace, gather);
-    else if (bits == 7) launch_pass<7>(capacity, persist, small_tiles, s, src_keys, sv, dk, dv, d_count, bits * p, sc.ghist + 256 * p, lb, sc.tickets + p, trace, gather);
-    else launch_pass<8>(capacity, persist, small_tiles, s, src_keys, sv, dk, dv, d_count, bits * p, sc.ghist + 256 * p, lb, sc.tickets + p, trace, gather);
+    if (bits == 5) launch_pass<5>(capacity, persist, s, src_keys, sv, dk, dv, d_count, bits * p, sc.ghist + 256 * p, lb, sc.tickets + p, gather);
+    else if (bits == 6) launch_pass<6>(capacity, persist, s, src_keys, sv, dk, dv, d_count, bits * p, sc.ghist + 256 * p, lb, sc.tickets + p, gather);
+    else if (bits == 7) launch_pass<7>(capacity, persist, s, src_keys, sv, dk, dv, d_count, bits * p, sc.ghist + 256 * p, lb, sc.tickets + p, gather);
+    else launch_pass<8>(capacity, persist, s, src_keys, sv, dk, dv, d_count, bits * p, sc.ghist + 256 * p, lb, sc.tickets + p, gather);
     uint32_t *t = sk; sk = dk; dk = t;
     t = sv; sv = dv; dv = t;
   }
   if (pass_events) cudaEventRecord(pass_events[passes], s);
-  if (trace_path && passes == 4) {
-    cudaStreamSynchronize(s);
-    uint64_t *h = (uint64_t *)malloc((size_t)tiles * 64);
-    cudaMemcpy(h, g_trace, (size_t)tiles * 64, cudaMemcpyDeviceToHost);
-    FILE *f = fopen(trace_path, "wb");
-    if (f) { fwrite(h, 64, tiles, f); fclose(f); }
-    free(h);
-  }
 }
 
 }  // namespace gs
